@@ -21,6 +21,11 @@ other BASELINE.json configurations and reports them as extra keys of the one JSO
             available) on a bounded sample of the same inputs, all host threads
 
 --impl reference  times that CPU restatement alone (same metric/config keys).
+
+--steps K sets the number of timed steps of every measurement above.  --dump-outputs DIR writes, after the timed
+steps, what the last one returned to its caller (ML-KEM: ct.npy, ss.npy; ML-DSA-65: sig.npy) as float32, one row per
+operation, for a fixed seeded sample of the operations whose global indices are in row_index.npy (float64).  The
+inputs depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -36,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree
 
 Q = 3329
 WORKLOADS = {
@@ -55,6 +61,7 @@ SM_HZ = 1.965e9
 # profiles/r02_ubench_keccak.txt), 148 SMs x 4 sub-partitions
 KECCAK_INSTR = 24 * 180
 KECCAK_PEAK = 148 * 4 * 0.5 * 32 * SM_HZ / KECCAK_INSTR
+DUMP_BYTES = 32 << 20  # --dump-outputs: at most this many bytes of float32 output rows
 
 
 def env_int(name, default):
@@ -94,6 +101,23 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback"
+
+
+def dump_rows(total: int, row_bytes: int):
+    """Global operation indices --dump-outputs writes: all of them if their rows fit DUMP_BYTES as float32, else a
+    fixed seeded sample, sorted."""
+    import numpy as np
+    k = min(total, DUMP_BYTES // (4 * row_bytes))
+    return np.sort(np.random.default_rng(0).choice(total, size=k, replace=False))
+
+
+def dump_outputs(out_dir: str, rows, arrays: dict):
+    """rows: the global indices of the dumped operations; arrays: name -> (len(rows), ...) output rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "row_index.npy"), np.asarray(rows, dtype=np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def mlkem_config(wl, n):
@@ -446,7 +470,7 @@ class Ctx:
 
 # ---------------------------------------------------------------- ML-KEM encaps (configs 3 and 5)
 def bench_mlkem(cx: Ctx, wl_key: str, log2n: int, steps: int, warmup: int, with_profile=True, with_cpu=True,
-                e2e_steps=5, sampler=None):
+                e2e_steps=5, sampler=None, dump_dir=None):
     import numpy as np
     torch, L, check = cx.torch, cx.L, cx.check
     from circl_b200 import mlkem
@@ -499,6 +523,12 @@ def bench_mlkem(cx: Ctx, wl_key: str, log2n: int, steps: int, warmup: int, with_
     ms_step = cx.max_over_ranks(ev0.elapsed_time(ev1) / steps)
     scheme.check_last_status()
     clocks = sampler.stop() if (sampler is not None and rank == 0) else None
+    if dump_dir is not None and rank == 0:
+        # N > 1: the caller of the gathered path receives every rank's rows in rank 0's buffer
+        ct_all, ss_all = (pg.matrix(0), pg.matrix(1)) if pg is not None else (ct_d, ss_d)
+        rows = dump_rows(world * n, wl["ct"] + 32)
+        sel = torch.as_tensor(rows, device=ct_all.device)
+        dump_outputs(dump_dir, rows, {"ct": ct_all[sel].cpu().numpy(), "ss": ss_all[sel].cpu().numpy()})
 
     # ---- N > 1: parity of the GATHERED buffer, the same step without the gather, and the gather alone
     gather = None
@@ -691,7 +721,7 @@ def bench_ntt(cx: Ctx, steps: int, warmup: int, with_cpu: bool):
         return cx.max_over_ranks(statistics.median(a.elapsed_time(b) for a, b in ts))
 
     for label, fn in (("forward", kyber.ntt_), ("inverse", kyber.inv_ntt_)):
-        ms = timed(fn, pristine, max(steps, 10))
+        ms = timed(fn, pristine, steps)
         gbs = npoly * 1024 / (ms * 1e-3) / 1e9
         ntt[label] = {"value": cx.world * npoly / (ms * 1e-3), "unit": "NTT/s", "ms_per_step": ms,
                       "roofline": {"bound": "hbm", "achieved": gbs, "peak": cx.peak, "unit": "GB/s",
@@ -700,7 +730,7 @@ def bench_ntt(cx: Ctx, steps: int, warmup: int, with_cpu: bool):
         if any16 is None:
             g = torch.Generator(device="cuda").manual_seed(1 + cx.rank)
             any16 = torch.randint(-32768, 32768, (npoly, 256), device="cuda", dtype=torch.int32, generator=g).to(torch.int16)
-        ms_any = timed(fn, any16, 5)
+        ms_any = timed(fn, any16, steps)
         ntt[label]["any_int16_inputs"] = {"ms_per_step": ms_any, "value": cx.world * npoly / (ms_any * 1e-3),
                                           "frac": npoly * 1024 / (ms_any * 1e-3) / 1e9 / cx.peak}
     del pristine, flush, any16
@@ -710,11 +740,11 @@ def bench_ntt(cx: Ctx, steps: int, warmup: int, with_cpu: bool):
                            "kernel reads and writes every byte once"}
     host_src = polys_h.clone()
     e2e_s = []
-    for i in range(5):
+    for i in range(warmup + steps):
         polys_h.copy_(host_src)
         t0 = time.perf_counter()
         check(L.cb200_kyber_ntt(polys_h.data_ptr(), npoly, 0))
-        if i >= 2:
+        if i >= warmup:
             e2e_s.append(time.perf_counter() - t0)
     del host_src
     ntt["e2e"] = {"value": cx.world * npoly / (sum(e2e_s) / len(e2e_s)), "unit": "NTT/s",
@@ -741,7 +771,7 @@ def bench_keccak(cx: Ctx, steps: int, warmup: int):
     for _ in range(warmup):
         keccak.permute_(st)
     cx.barrier()
-    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(max(steps, 8))]
+    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for a, b in evs:
         a.record()
         keccak.permute_(st)
@@ -762,7 +792,7 @@ def bench_keccak(cx: Ctx, steps: int, warmup: int):
 
 
 # ---------------------------------------------------------------- ML-DSA-65 (BASELINE configs[3])
-def bench_mldsa(cx: Ctx, log2n: int, steps: int, warmup: int, with_cpu: bool, sampler=None):
+def bench_mldsa(cx: Ctx, log2n: int, steps: int, warmup: int, with_cpu: bool, sampler=None, dump_dir=None):
     import numpy as np
     torch, L, check = cx.torch, cx.L, cx.check
     rank, world = cx.rank, cx.world
@@ -806,13 +836,16 @@ def bench_mldsa(cx: Ctx, log2n: int, steps: int, warmup: int, with_cpu: bool, sa
     clocks = sampler.stop() if (sampler is not None and rank == 0) else None
     att = attempts.value / n
     assert int(st_d.sum().item()) == 0
+    if dump_dir is not None and rank == 0:
+        # each rank signs its own shard; rank 0's caller receives rank 0's signatures
+        rows = dump_rows(n, 3309)
+        dump_outputs(dump_dir, rows, {"sig": sig_d[torch.as_tensor(rows, device=sig_d.device)].cpu().numpy()})
     step_host()
     cx.barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(steps, 3))
-    for _ in range(e2e_steps):
+    for _ in range(steps):
         step_host()
-    e2e_ms = cx.max_over_ranks(1e3 * (time.perf_counter() - t0) / e2e_steps)
+    e2e_ms = cx.max_over_ranks(1e3 * (time.perf_counter() - t0) / steps)
     same = bool(torch.equal(sig_h[:4096], sig_d[:4096].cpu()))
     kernels = cx.profile(step_device)
     tot = sum(v["ms_total"] for v in kernels.values())
@@ -865,7 +898,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ntt", action="store_true", help="skip the secondary NTT / Keccak measurements")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra BASELINE configs (mldsa65 at N = 1, mlkem1024 at N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (a fixed sample of its rows) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -878,10 +917,11 @@ def main():
               "vs_baseline": None, "data": "synthetic"}
     if args.workload == "mldsa65":
         log2 = args.batch_log2 if args.batch_log2 != 20 else 18
-        rec, clocks = bench_mldsa(cx, log2, args.steps, args.warmup, with_cpu, sampler)
+        rec, clocks = bench_mldsa(cx, log2, args.steps, args.warmup, with_cpu, sampler, args.dump_outputs)
         line = dict(rec, **common, clocks=clocks)
     else:
-        rec, clocks = bench_mlkem(cx, args.workload, args.batch_log2, args.steps, args.warmup, True, with_cpu, 5, sampler)
+        rec, clocks = bench_mlkem(cx, args.workload, args.batch_log2, args.steps, args.warmup, True, with_cpu, args.steps,
+                                  sampler, args.dump_outputs)
         line = dict(rec, **common, dtype="int16", clocks=clocks)
         line.pop("per_gpu", None)
         if not args.no_ntt:
@@ -889,11 +929,11 @@ def main():
             line["keccak"] = bench_keccak(cx, args.steps, args.warmup)
         if not args.no_extras and args.workload == "mlkem768" and args.batch_log2 == 20:
             if cx.world == 1:
-                line["mldsa65"], _ = bench_mldsa(cx, 18, min(args.steps, 5), 3, with_cpu)
+                line["mldsa65"], _ = bench_mldsa(cx, 18, args.steps, 3, with_cpu)
             else:
                 # BASELINE configs[4]: 2^21 per GPU = 2^24 over 8 GPUs, gathered to rank 0 (26.8 GB at N = 8)
-                line["mlkem1024"], _ = bench_mlkem(cx, "mlkem1024", 21, min(args.steps, 5), 3, with_profile=False,
-                                                   with_cpu=False, e2e_steps=2)
+                line["mlkem1024"], _ = bench_mlkem(cx, "mlkem1024", 21, args.steps, 3, with_profile=False,
+                                                   with_cpu=False, e2e_steps=args.steps)
     if cx.rank == 0:
         print(json.dumps(line))
     if cx.world > 1:

@@ -1,5 +1,6 @@
 import gzip
 import json
+import lzma
 import os
 import sys
 
@@ -17,7 +18,7 @@ def pytest_configure(config):
 
 
 def load_golden(name):
-    with gzip.open(os.path.join(GOLDEN, name)) as f:
+    with (lzma.open if name.endswith(".xz") else gzip.open)(os.path.join(GOLDEN, name)) as f:
         return json.load(f)
 
 
@@ -48,4 +49,4 @@ def mldsa_other_acvp():
 
 @pytest.fixture(scope="session")
 def mldsa_wycheproof():
-    return load_golden("mldsa_wycheproof.json.gz")
+    return load_golden("mldsa_wycheproof.json.xz")

@@ -2,8 +2,8 @@
 """Extract the reference's own fixtures for the module-lattice hot path into
 small committed files under tests/golden/.
 
-Run in the build container (needs /root/reference; the GPU box does not have
-it):   python tests/golden/make_golden.py
+Needs a checkout of cloudflare/circl; the tests read only the files written here:
+       python tests/golden/make_golden.py <path to the circl checkout>
 
 Nothing here executes reference code (it is Go; there is no Go toolchain).  It
 only re-packages the reference's test DATA:
@@ -15,11 +15,13 @@ only re-packages the reference's test DATA:
 """
 import gzip
 import json
+import lzma
 import os
 import re
+import sys
 import zlib
 
-REF = "/root/reference"
+REF = None  # the circl checkout, set from the command line
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -40,8 +42,12 @@ def acvp(sub_dir):
 def dump(name, obj):
     raw = json.dumps(obj, separators=(",", ":"), sort_keys=True).encode()
     path = os.path.join(OUT, name)
-    with gzip.GzipFile(path, "wb", mtime=0) as f:
-        f.write(raw)
+    if name.endswith(".xz"):  # for the fixtures gzip would leave above 1 MB
+        with open(path, "wb") as f:
+            f.write(lzma.compress(raw, preset=9 | lzma.PRESET_EXTREME))
+    else:
+        with gzip.GzipFile(path, "wb", mtime=0) as f:
+            f.write(raw)
     print(f"{name}: {os.path.getsize(path)} bytes")
 
 
@@ -214,7 +220,7 @@ def wycheproof():
                     o[k] = g[k]
             groups.append(o)
         out[f.replace(".json.gz", "")] = {"algorithm": ts["algorithm"], "groups": groups}
-    dump("mldsa_wycheproof.json.gz", out)
+    dump("mldsa_wycheproof.json.xz", out)
 
 
 def keccak_kats():
@@ -233,6 +239,9 @@ def keccak_kats():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    REF = sys.argv[1]
     mlkem()
     mldsa65()
     mldsa_other()
