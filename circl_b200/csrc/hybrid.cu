@@ -436,7 +436,7 @@ int cb200_xwing_encaps(const uint8_t* pk, size_t pk_stride, const uint8_t* eseed
                        size_t n) {
   int rc = require_ready();
   if (rc) return rc;
-  if (!pk || !eseeds || !ct || !ss || (pk_stride != 0 && pk_stride < 1216) || (pk_stride & 15)) {
+  if (!pk || !eseeds || !ct || !ss || (pk_stride != 0 && pk_stride < 1216)) {
     set_error("cb200_xwing_encaps: bad argument");
     return CB200_ERR_ARG;
   }
@@ -448,7 +448,7 @@ int cb200_xwing_encaps(const uint8_t* pk, size_t pk_stride, const uint8_t* eseed
   }
   if (dev) {
     if (!aligned16({pk, eseeds, ct, ss}, {pk_stride})) {
-      set_error("cb200_xwing_encaps: device buffers must be 16-byte aligned");
+      set_error("cb200_xwing_encaps: device buffers and pk_stride must be 16-byte aligned");
       return CB200_ERR_ARG;
     }
     DeviceCall call(ct);
@@ -474,7 +474,7 @@ int cb200_xwing_encaps(const uint8_t* pk, size_t pk_stride, const uint8_t* eseed
 int cb200_xwing_decaps(const uint8_t* sk, size_t sk_stride, const uint8_t* ct, uint8_t* ss, size_t n) {
   int rc = require_ready();
   if (rc) return rc;
-  if (!sk || !ct || !ss || (sk_stride != 0 && sk_stride < 32) || (sk_stride & 3)) {
+  if (!sk || !ct || !ss || (sk_stride != 0 && sk_stride < 32)) {
     set_error("cb200_xwing_decaps: bad argument");
     return CB200_ERR_ARG;
   }
@@ -548,7 +548,7 @@ int cb200_hybrid_encaps(int id, const uint8_t* pk, size_t pk_stride, const uint8
   int rc = require_ready();
   if (rc) return rc;
   Hyb H;
-  if (!hyb_of(id, &H) || !pk || !seeds || !ct || !ss || (pk_stride != 0 && pk_stride < H.ek + 32) || (pk_stride & 15)) {
+  if (!hyb_of(id, &H) || !pk || !seeds || !ct || !ss || (pk_stride != 0 && pk_stride < H.ek + 32)) {
     set_error("cb200_hybrid_encaps: bad argument");
     return CB200_ERR_ARG;
   }
@@ -564,7 +564,7 @@ int cb200_hybrid_encaps(int id, const uint8_t* pk, size_t pk_stride, const uint8
       return CB200_ERR_ARG;
     }
     if (!aligned16({pk, seeds, ct, ss}, {pk_stride})) {
-      set_error("cb200_hybrid_encaps: device buffers must be 16-byte aligned");
+      set_error("cb200_hybrid_encaps: device buffers and pk_stride must be 16-byte aligned");
       return CB200_ERR_ARG;
     }
     DeviceCall call(ct);
@@ -592,7 +592,7 @@ int cb200_hybrid_decaps(int id, const uint8_t* sk, size_t sk_stride, const uint8
   int rc = require_ready();
   if (rc) return rc;
   Hyb H;
-  if (!hyb_of(id, &H) || !sk || !ct || !ss || sk_stride < H.dk + 32 || (sk_stride & 15)) {
+  if (!hyb_of(id, &H) || !sk || !ct || !ss || sk_stride < H.dk + 32) {
     set_error("cb200_hybrid_decaps: bad argument (one decapsulation key per operation: sk_stride >= key size)");
     return CB200_ERR_ARG;
   }
@@ -607,8 +607,8 @@ int cb200_hybrid_decaps(int id, const uint8_t* sk, size_t sk_stride, const uint8
       set_error("cb200_hybrid_decaps: device-pointer calls need a status array (it carries kem.ErrPubKey / kem.ErrPrivKey)");
       return CB200_ERR_ARG;
     }
-    if (!aligned16({sk, ct, ss}, {})) {
-      set_error("cb200_hybrid_decaps: device buffers must be 16-byte aligned");
+    if (!aligned16({sk, ct, ss}, {sk_stride})) {
+      set_error("cb200_hybrid_decaps: device buffers and sk_stride must be 16-byte aligned");
       return CB200_ERR_ARG;
     }
     DeviceCall call(ss);

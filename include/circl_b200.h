@@ -6,7 +6,11 @@
  * pointers and sizes only.  Every buffer is caller-owned and never retained
  * past the call.  A pointer may be a host pointer (pageable or pinned) or a
  * CUDA device pointer; the library detects which (cudaPointerGetAttributes)
- * and stages host buffers through HBM itself.  All entry points return 0 on
+ * and stages host buffers through HBM itself.  Where a call takes a row stride
+ * (op i uses base + i*stride), a host-pointer stride may be any value at least
+ * the row size; device-pointer calls of the KEM and signature entry points
+ * want their buffers and key strides 16-byte aligned (CB200_ERR_ARG
+ * otherwise).  All entry points return 0 on
  * success or a negative code; cb200_last_error() gives the message.  There is
  * no CPU fallback: without a usable CUDA device every compute call fails.
  *
